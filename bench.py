@@ -151,6 +151,51 @@ def _layout(sizes):
     return offs, pos
 
 
+DUMP_MAX_BLOBS = 1 << 18            # 32 MiB of float32 digests; larger batches are sampled
+DUMP_CACHE_BLOBS, DUMP_CACHE_BYTES = 256, 4096
+
+
+def dump_outputs(out_dir, eng, digests, matched, sizes, blob_ids, cached, prefix=""):
+    """What the timed step returned, as float32/float64 .npy files under out_dir, so that two builds run with the
+    same arguments (hence the same seeded inputs) can be compared output for output:
+      digests.npy      (k, 32) float32  the SHA-256 of each blob, one byte per value
+      matched.npy      (k,)    float32  1 where the digest equalled the expected one
+      blob_index.npy   (k,)    float64  which synthetic blob each row is (all of them up to DUMP_MAX_BLOBS, else a
+                                        fixed seeded sample)
+      cache_sample.npy (m,)    float32  bytes read back from the CAS through the hit path (dm_cache_open/read), a
+                                        window of up to DUMP_CACHE_BYTES in each of up to DUMP_CACHE_BLOBS blobs;
+                                        hash-and-cache mode only
+      cache_sample_at.npy (b, 3) float64  (blob index, offset, length) of each window in cache_sample.npy
+    At most about 39 MiB in all.  With N > 1 GPUs each rank writes its own set, its names prefixed rank<r>_."""
+    import numpy as np
+    n = len(sizes)
+    rng = np.random.default_rng(SEED)
+    rows = np.arange(n) if n <= DUMP_MAX_BLOBS else np.sort(rng.choice(n, DUMP_MAX_BLOBS, replace=False))
+    blob_ids = np.asarray(blob_ids, dtype=np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(name, arr):
+        np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), arr)
+    save("digests", np.asarray(digests).reshape(n, 32)[rows].astype(np.float32))
+    save("matched", np.asarray(matched)[rows].astype(np.float32))
+    save("blob_index", blob_ids[rows])
+    if not cached:
+        return
+    picks = rows if len(rows) <= DUMP_CACHE_BLOBS else np.sort(rng.choice(rows, DUMP_CACHE_BLOBS, replace=False))
+    at, parts = [], []
+    for r in picks:
+        ln = min(DUMP_CACHE_BYTES, int(sizes[r]))
+        off = int(rng.integers(0, int(sizes[r]) - ln + 1))
+        rid, _ = eng.cache_open(np.asarray(digests)[32 * r:32 * r + 32].tobytes())
+        try:
+            parts.append(np.frombuffer(eng.cache_read(rid, off, ln), dtype=np.uint8))
+        finally:
+            eng.cache_close(rid)
+        at.append((blob_ids[r], off, ln))
+    save("cache_sample", np.concatenate(parts).astype(np.float32) if parts else np.zeros(0, dtype=np.float32))
+    save("cache_sample_at", np.asarray(at, dtype=np.float64).reshape(-1, 3))
+
+
 def _my_blob_indices(n_blobs, rank, world):
     """Disjoint per-rank blob sets chosen by the production router: synthetic
     blobs have no digest before they are hashed, so they are homed by URL hash
@@ -333,7 +378,11 @@ def main():
     ap.add_argument("--cas-slack-mib", type=int, default=4096, help="HBM arena beyond one copy of the workload (ring-path bodies, probes)")
     ap.add_argument("--blobs", type=int, default=0, help="override: number of blobs (with --blob-bytes)")
     ap.add_argument("--blob-bytes", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.blobs and args.blob_bytes:
         args.workload = f"custom_{args.blobs}x{args.blob_bytes}"
         WORKLOADS[args.workload] = {"sizes": [args.blob_bytes] * args.blobs, "baseline_config": None}
@@ -427,6 +476,9 @@ def main():
     s1 = eng.stats()
     assert np.array_equal(d, expect_arr) and m.all()
     launches = int(s1["kernel_launches"] - s0["kernel_launches"])
+    if args.dump_outputs:                               # before the later legs evict what the timed steps cached
+        dump_outputs(args.dump_outputs, eng, d, m, sizes, mine, cached=not args.hash_only,
+                     prefix="" if world == 1 else f"rank{rank}_")
 
     tt = torch.tensor([wall, kernel_ms], dtype=torch.float64, device=f"cuda:{local}")
     if world > 1:
@@ -503,7 +555,7 @@ def main():
 
     # small-blob latency through the stream API: open -> write 4 KiB -> finish (DMA + launch + digest back)
     if probes is not None:
-        small = np.frombuffer(os.urandom(4096), dtype=np.uint8)
+        small = np.random.default_rng(SEED).integers(0, 256, 4096, dtype=np.uint8)
         lat = []
         for it in range(220):
             t0_ = time.perf_counter()
